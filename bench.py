@@ -248,6 +248,21 @@ def bind_to_gpu_numa(local):
     return info
 
 
+DUMP_STREAMS = 64          # 64 streams x 2 pictures x 101,376 samples x 4 bytes = 52 MB
+
+
+def dump_outputs(ctx, out_dir, streams):
+    """What the last timed step left in the frame store, as a caller of ef_decode_all reads it back: the last and
+    the second-to-last picture (I420) of a fixed, seeded sample of this rank's streams, in stream order, as float32
+    arrays DIR/frames_last.npy and DIR/frames_prev.npy of shape (min(64, streams), 101376)."""
+    os.makedirs(out_dir, exist_ok=True)
+    sample = np.sort(np.random.default_rng(0).choice(streams, size=min(DUMP_STREAMS, streams), replace=False))
+    last = np.stack([ctx.read_frame_i420(int(i), -1) for i in sample])
+    prev = np.stack([ctx.read_frame_i420(int(i), ((ctx.stream_info(int(i))[1] + PICTURES) & 1) ^ 1) for i in sample])
+    np.save(os.path.join(out_dir, "frames_last.npy"), last.astype(np.float32))
+    np.save(os.path.join(out_dir, "frames_prev.npy"), prev.astype(np.float32))
+
+
 def run_gpu(args):
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     if args.gpus > 1 and world == 1:       # convenience: re-launch under torchrun
@@ -353,8 +368,6 @@ def run_gpu(args):
     ctx.submit_es(dev_es.data_ptr(), dev_off.data_ptr(), st, device=True)
     for _ in range(args.warmup):
         step_resident()
-    info = ctx.index_info()
-    assert info["total_pictures"] == streams * PICTURES, info
 
     sampler = ClockSampler(local)
     if rank == 0:
@@ -371,6 +384,10 @@ def run_gpu(args):
     launches = ctx.launch_count() - launches0
     ms_total = t0.elapsed_time(t1)
     k1_ms = sum(ev[k][0].elapsed_time(ev[k][1]) for k in range(args.steps))
+    info = ctx.index_info()
+    assert info["total_pictures"] == streams * PICTURES, info
+    if args.dump_outputs and rank == 0:
+        dump_outputs(ctx, args.dump_outputs, streams)
 
     # --verify (checker only, after the timed region): this rank's first distinct streams through the oracle
     verified = None
@@ -583,7 +600,13 @@ def main():
     ap.add_argument("--no-e2e-all", action="store_true", help="skip the all-pictures read-back leg (5 GB pinned per GPU)")
     ap.add_argument("--no-e2e-ts", action="store_true", help="skip the transport-stream input leg")
     ap.add_argument("--no-numa", action="store_true", help="do not pin the rank to its GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the decoded pictures of the last step "
+                    "(last two pictures of 64 seeded-sampled streams of rank 0) to DIR as float32 .npy files")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's pictures; --impl reference has none")
     args.warmup = max(args.warmup, 0)
     import __graft_entry__
     if not os.path.exists(os.path.join(ROOT, "espflix_b200", "libespflix_b200.so")):

@@ -1,10 +1,9 @@
 """Audio path on the CPU (SURVEY.md 8f-3): the oracle restatement (oracle/ef_oracle_audio.c) against the pins the
-unmodified reference produced on its own fixtures (tests/golden/audio_pins.json, tools/make_audio_golden.py), against
-the reference itself on synthetic transport streams (wherever oracle/_ref exists), and the constant tables."""
+unmodified reference produced on its own fixtures (tests/golden/audio_pins.json, tools/make_audio_golden.py) and on
+synthetic transport streams (tests/golden/ref_pins.json, tools/make_ref_golden.py), and the constant tables."""
 import hashlib
 import json
 import os
-import subprocess
 
 import numpy as np
 import pytest
@@ -13,7 +12,6 @@ from tests import audio_cases
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 G = os.path.join(ROOT, "tests", "golden")
-REF_AUDIO = os.path.join(ROOT, "oracle", "_ref", "efref_audio")
 
 
 def _masked(pcm, ranges):
@@ -53,26 +51,33 @@ def test_sbc_tables_match_reference_arrays():
     assert table("ef_sbc_offset8[4][8]") == g["SBC_offset8"]
 
 
-@pytest.mark.skipif(not os.path.exists(REF_AUDIO), reason="oracle/_ref not built (no /root/reference here)")
-@pytest.mark.parametrize("case", ["bp28", "snr_bp12_f0", "bp60_loud", "rejected_frames", "muted_pes", "pid102"])
-def test_oracle_matches_reference_on_synthetic_streams(oracle, tmp_path, case):
-    kw = {"bp28": dict(bitpool=28), "snr_bp12_f0": dict(bitpool=12, allocation=1, frequency=0), "bp60_loud": dict(bitpool=60, loud=True, frequency=3),
-          "rejected_frames": dict(bitpool=28, bad_frames=(3, 4, 17)), "muted_pes": dict(bitpool=28), "pid102": dict(bitpool=28, frequency=1)}[case]
-    es = audio_cases.sbc_stream(1000 + len(case), 40, **kw)
+SYNTHETIC_CASES = {"bp28": dict(bitpool=28), "snr_bp12_f0": dict(bitpool=12, allocation=1, frequency=0), "bp60_loud": dict(bitpool=60, loud=True, frequency=3),
+                   "rejected_frames": dict(bitpool=28, bad_frames=(3, 4, 17)), "muted_pes": dict(bitpool=28), "pid102": dict(bitpool=28, frequency=1)}
+
+
+def synthetic_stream(case):
+    """(SBC stream, its transport stream) of one synthetic case"""
+    es = audio_cases.sbc_stream(1000 + len(case), 40, **SYNTHETIC_CASES[case])
     ts = audio_cases.mux_audio_ts(es, pid=0x102 if case == "pid102" else 0x101, drop_pts_on=(1,) if case == "muted_pes" else ())
-    p = tmp_path / "a.ts"
-    p.write_bytes(ts.tobytes())
-    out = tmp_path / "a.bin"
-    subprocess.run([REF_AUDIO, str(p), str(out)], check=True, capture_output=True, timeout=120)   # one process per run: the reference keeps its state in globals
-    raw = out.read_bytes()
-    nes, npcm = [int(x) for x in np.frombuffer(raw[:16], dtype=np.uint64)]
-    ref_es = np.frombuffer(raw[16:16 + nes], dtype=np.uint8)
-    ref_pcm = np.frombuffer(raw[16 + nes:16 + nes + 2 * npcm], dtype=np.int16)
-    ref_pdm = np.frombuffer(raw[16 + nes + 2 * npcm:], dtype=np.uint16)
+    return es, ts
+
+
+def _sha(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+@pytest.mark.parametrize("case", list(SYNTHETIC_CASES))
+def test_oracle_matches_reference_on_synthetic_streams(oracle, case):
+    """The reference's demux -> decode_audio -> PDM output on each stream is pinned in tests/golden/ref_pins.json
+    (tools/make_ref_golden.py)."""
+    pin = json.load(open(os.path.join(G, "ref_pins.json")))["audio"][case]
+    es, ts = synthetic_stream(case)
+    assert _sha(ts) == pin["in_sha256"], "synthetic stream %s changed" % case
     got_es = oracle.demux_audio_ts(ts)
-    assert np.array_equal(got_es, ref_es)
+    assert got_es.size == pin["es_bytes"] and _sha(got_es) == pin["es_sha256"]
     if case == "muted_pes":
         assert got_es.size == es.size - 1024              # the second PES (no PTS) is dropped whole; the third one opens the stream again
     pcm = oracle.sbc_decode(got_es)
-    assert npcm > 0 and np.array_equal(pcm, ref_pcm)
-    assert np.array_equal(oracle.pdm(pcm), ref_pdm)
+    assert pin["pcm_samples"] > 0 and pcm.size == pin["pcm_samples"] and _sha(pcm) == pin["pcm_sha256"]
+    pdm = oracle.pdm(pcm)
+    assert pdm.size == pin["pdm_words"] and _sha(pdm) == pin["pdm_sha256"]

@@ -1,13 +1,13 @@
 """PTS -> field pacing of push_video (SURVEY.md 8f-2; video.cpp:1023-1057, 1165-1177), CPU side: the C restatement
-of the schedule against the pins the unmodified reference produced (tools/make_pacing_golden.py) and, where
-oracle/_ref exists, against the reference itself (real push_video / video_isr on two threads) for irregular PTS."""
+of the schedule against the pins the unmodified reference produced (tools/make_pacing_golden.py), and against what
+the reference itself (real push_video / video_isr on two threads) produced for irregular PTS (tools/make_ref_golden.py)."""
 import json
 import os
 
 import numpy as np
 import pytest
 
-from tests.oracle_lib import Oracle, RefVideo, have_ref
+from tests.oracle_lib import Oracle
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PINS = json.load(open(os.path.join(ROOT, "tests", "golden", "pacing_pins.json")))
@@ -22,23 +22,15 @@ def test_schedule_matches_reference_pins(name):
     assert hs.tolist() == p["hscroll"]                    # the poster scroll (_animate / _easd) field by field
 
 
-@pytest.mark.skipif(not have_ref(), reason="oracle/_ref not built (needs /root/reference)")
 def test_schedule_matches_reference_on_irregular_pts():
-    """Jitter, repeated and decreasing PTS (late frames, 'resetting v timing'), long gaps, both standards."""
-    o, rv = Oracle(), RefVideo()
-    rng = np.random.default_rng(2024)
-    frames = np.zeros((2, 101376), dtype=np.uint8)                      # content is irrelevant to the schedule
-    for case in range(24):
-        ntsc = case % 2
-        n = int(rng.integers(2, 14))
-        step = rng.choice([3003, 3003, 3003, 1501, 6006, 0, -4000, 45045], size=n)
-        pts = (129003 + np.cumsum(step)).astype(np.int64)
-        pts = np.maximum(pts, 0)
-        fc0 = int(rng.integers(0, 4)) if case < 8 else int(rng.integers(1, 100000))
-        fr = np.ascontiguousarray(np.broadcast_to(frames[0], (n, 101376)))
-        modes = np.where(rng.random(n) < 0.2, rng.integers(1, 4, size=n), 0).astype(np.int32)      # 1 at once, 2 / 3 poster scroll
-        tail = int(rng.integers(0, 20))
-        rf, rff, rfl, _, rhs = rv.paced(fr, pts, ntsc, fc0, 400, want_fields=False, modes=modes, tail_fields=tail, want_hscroll=True)
-        f, ff, fl, hs = o.paced_schedule(pts, ntsc, fc0, 400, modes=modes, tail_fields=tail, want_hscroll=True)
-        assert (f, ff.tolist(), fl.tolist()) == (rf, rff.tolist(), rfl.tolist()), (case, ntsc, fc0, pts.tolist())
-        assert hs.tolist() == rhs.tolist(), (case, modes.tolist())
+    """Jitter, repeated and decreasing PTS (late frames, 'resetting v timing'), long gaps, both standards: the
+    schedules the reference's real push_video / video_isr produced for these PTS lists, pinned with them in
+    tests/golden/ref_pins.json (tools/make_ref_golden.py)."""
+    o = Oracle()
+    cases = json.load(open(os.path.join(ROOT, "tests", "golden", "ref_pins.json")))["pacing"]
+    assert len(cases) == 24
+    for case, p in enumerate(cases):
+        pts = np.array(p["pts"], dtype=np.int64)
+        f, ff, fl, hs = o.paced_schedule(pts, p["ntsc"], p["frame_counter0"], p["max_fields"], modes=p["modes"], tail_fields=p["tail_fields"], want_hscroll=True)
+        assert (f, ff.tolist(), fl.tolist()) == (p["fields"], p["flip_field"], p["flip_line"]), (case, p["ntsc"], p["frame_counter0"], p["pts"])
+        assert hs.tolist() == p["hscroll"], (case, p["modes"])
